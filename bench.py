@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a engine
     python bench.py --impl reference --gpus N --steps K ...   # the CPU restatement of the reference path
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's embeddings as .npy
 
 Workload (BASELINE.json configs[1]): text_sonar_basic_encoder architecture (24 layers, d=1024,
 16 heads, FFN 8192, vocab 256206, random-init weights), batch 4096 sentences x 128 tokens of
@@ -58,6 +59,22 @@ def kernel_source_digest() -> str:
         with open(os.path.join(ROOT, "sonar_b200", "csrc", name), "rb") as f:
             h.update(f.read())
     return h.hexdigest()[:16]
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, name: str, t: torch.Tensor) -> None:
+    """Write `t` as `path/<name>.npy` in float32.  An output larger than 64 MB is cut to a fixed sample of its rows (seed 0,
+    sorted), the same rows from run to run, so that dumps of two builds compare row for row."""
+    import numpy as np
+
+    a = t.detach().float().cpu()
+    keep = DUMP_BYTES // (a[0].numel() * 4)
+    if a.shape[0] > keep:
+        a = a[torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, name + ".npy"), a.numpy())
 
 
 def load_peaks():
@@ -220,8 +237,10 @@ def run_reference(args):
         enc(ids, None)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        enc(ids, None)
+        emb, _ = enc(ids, None)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "sentence_embeddings", emb)
     val = per_step * args.steps / dt
     line = {
         "impl": "reference", "metric": "sentences/sec->1024-d", "value": val, "unit": "sentences/s",
@@ -647,6 +666,10 @@ def main():
     ap.add_argument("--config5-per-gpu", type=int, default=125000, help="sentences every rank encodes for config 5")
     ap.add_argument("--layers", type=int, default=0, help="--impl reference only: reduced depth for the CPU test-suite")
     ap.add_argument("--vocab", type=int, default=0, help="--impl reference only: reduced vocabulary for the CPU test-suite")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the sentence embeddings of the last timed step as "
+                         "DIR/sentence_embeddings.npy (float32; with N > 1 the all-gathered [N*batch,1024]; above 64 MB "
+                         "a fixed seeded sample of rows)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -699,6 +722,7 @@ def main():
         out = model(batch_dev).sentence_embeddings
         if dist is not None:  # the one exchange step of the path: assemble [N,1024] on every rank
             dist.all_gather_into_tensor(gather_buf, out)
+            return gather_buf
         return out
 
     out_host = torch.empty((B, D), dtype=torch.float32).pin_memory()
@@ -722,8 +746,9 @@ def main():
             sampler.start()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
+        out = None
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         torch.cuda.synchronize()
         if dist is not None:
@@ -733,7 +758,7 @@ def main():
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if dist is not None:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item()), clocks
+        return float(ms.item()), clocks, out
 
     # dominant kernel timed INSIDE the real steps: events recorded by the engine around the middle layer's FFN1 GEMM
     k_ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
@@ -744,7 +769,9 @@ def main():
     k_a = args.steps // 2
     k_b = args.steps - k_a
     e2e_a = timed(step_e2e, k_a, args.warmup)[0] if k_a else 0.0
-    total_ms, clocks = timed(step_resident, args.steps, args.warmup, sample_clocks=True)
+    total_ms, clocks, last_out = timed(step_resident, args.steps, args.warmup, sample_clocks=True)
+    if args.dump_outputs and rank == 0:  # now: the e2e steps below reuse gather_buf
+        dump_outputs(args.dump_outputs, "sentence_embeddings", last_out)
     in_step_kernel_ms = k_ev[0].elapsed_time(k_ev[1])  # the last timed step's launch
     model.profile_ffn1(None, None)
     e2e_b = timed(step_e2e, k_b, 1)[0]

@@ -258,23 +258,21 @@ def test_sampling_argument_errors():
 def test_sampler_subsets_equal_huggingface_logits_warpers():
     """Which tokens a sampler may draw -- the k most probable / the smallest most-probable-first set whose mass reaches p --
     against HuggingFace's TopKLogitsWarper / TopPLogitsWarper on random distributions (the random streams differ, the
-    subsets must not)."""
-    from transformers.generation.logits_process import TopKLogitsWarper, TopPLogitsWarper
-
+    subsets must not; the warpers' subsets are stored in tests/golden/logits_warpers_hf.pt, made by
+    tests/golden/make_logits_warpers_golden.py)."""
     from sonar_b200.sampling import TopKSampler, TopPSampler
 
-    g = torch.Generator().manual_seed(11)
-    logits = torch.randn((64, 16), generator=g) * 2.5
+    hf = torch.load(os.path.join(os.path.dirname(__file__), "golden", "logits_warpers_hf.pt"), weights_only=True)
+    logits = hf["logits"]
     probs = logits.softmax(1)
     order = torch.argsort(probs, dim=1, descending=True, stable=True)
     sorted_probs = torch.gather(probs, 1, order)
-    ids = torch.zeros((64, 1), dtype=torch.long)
     for k in (1, 3, 8, 14):
         w, _ = TopKSampler(k).weights(sorted_probs)
         kept = torch.zeros_like(probs, dtype=torch.bool).scatter_(1, order, w > 0)
-        assert torch.equal(kept, TopKLogitsWarper(top_k=k)(ids, logits.clone()) > float("-inf"))
+        assert torch.equal(kept, hf[f"top_k={k}"])
     for p in (0.3, 0.6, 0.9, 0.99):
         w, short = TopPSampler(p).weights(sorted_probs)
         kept = torch.zeros_like(probs, dtype=torch.bool).scatter_(1, order, w > 0)
-        assert torch.equal(kept, TopPLogitsWarper(top_p=p)(ids, logits.clone()) > float("-inf"))
+        assert torch.equal(kept, hf[f"top_p={p}"])
         assert not bool(short.any())  # the rows sum to 1 > p: the nucleus always closes inside the 16 candidates

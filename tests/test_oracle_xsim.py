@@ -1,13 +1,22 @@
 """The xsim oracle (oracle/xsim.py) against an INDEPENDENT implementation: scikit-learn's brute-force cosine k-NN for the
-neighbour search, and a literal dense evaluation of the LASER margin formula for the scoring.  The reference itself has no
-xsim code (README.md:5 names the task only), so this is the strongest pin available offline; CPU only."""
+neighbour search (its results on these seeded inputs are stored in tests/golden/xsim_sklearn_knn.pt, made by
+tests/golden/make_xsim_sklearn_golden.py), and a literal dense evaluation of the LASER margin formula for the scoring.  The
+reference itself has no xsim code (README.md:5 names the task only), so this is the strongest pin available offline; CPU only."""
+
+import os
 
 import numpy as np
 import pytest
+import torch
 
 from oracle import xsim as ox
 
-sk = pytest.importorskip("sklearn.neighbors")
+GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "xsim_sklearn_knn.pt")
+CASES = [(200, 300, 64, 4), (257, 129, 32, 5), (64, 64, 16, 1)]
+
+
+def case_key(n, m, d, k):
+    return f"n{n}_m{m}_d{d}_k{k}"
 
 
 def _data(n, m, d, seed, noise=0.3):
@@ -18,12 +27,18 @@ def _data(n, m, d, seed, noise=0.3):
     return x, y
 
 
-@pytest.mark.parametrize("n,m,d,k", [(200, 300, 64, 4), (257, 129, 32, 5), (64, 64, 16, 1)])
-def test_oracle_knn_equals_sklearn_brute_force_cosine(n, m, d, k):
+@pytest.fixture(scope="module")
+def sklearn_knn():
+    return torch.load(GOLDEN, weights_only=True)
+
+
+@pytest.mark.parametrize("n,m,d,k", CASES)
+def test_oracle_knn_equals_sklearn_brute_force_cosine(sklearn_knn, n, m, d, k):
     x, y = _data(n, m, d, seed=n + m)
     val, idx = ox.knn(x, y, k)
-    nn = sk.NearestNeighbors(n_neighbors=k, metric="cosine", algorithm="brute").fit(y.astype(np.float64))
-    dist, ind = nn.kneighbors(x.astype(np.float64))
+    ref = sklearn_knn[case_key(n, m, d, k)]
+    ind, dist = ref["indices"].numpy(), ref["distances"].numpy()
+    assert ind.shape == (n, k)
     assert np.array_equal(idx, ind)
     np.testing.assert_allclose(val, 1.0 - dist, rtol=0, atol=1e-12)
 
